@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Driver benchmark for the B200-native quantized-linear hot path.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME] [--no-extras]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME] [--no-extras] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input.  The default workload is the configuration
 BASELINE.json's metric is quoted on (configs[1]): the bf16 x int4 QLinear GEMM M=4096, K=4096, N=14336 (Llama-3-8B FFN
@@ -20,6 +20,10 @@ total work is fixed.  Outside the timed region every rank checks the gathered ou
 linear on the full weight and the line carries `"parity_ok"`.
 
 One JSON line is printed by rank 0 (see the keys in DESIGN.md "Measurement").
+
+`--dump-outputs DIR` also writes what the last timed step of every measured workload returned, as DIR/<workload>.npy in
+float32 (for M > 32 a fixed, seeded sample of rows; about 32 MB for the default run).  Every input comes from a fixed
+seed, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -73,6 +77,31 @@ def algorithmic(kind, M, N, K):
     else:
         byts = M * K + N * K + N * 2 + M * N * 2
     return flops, byts
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_rows(M):
+    """Rows of an [M, N] result that --dump-outputs writes: all of them up to M = 32, else two rows of every 32-row band
+    picked with a fixed seed (every M tile of every kernel is represented: 256 rows of M = 4096)."""
+    import numpy as np
+    if M <= 32:
+        return np.arange(M)
+    rng = np.random.default_rng(0)
+    return np.concatenate([b0 + np.sort(rng.choice(min(32, M - b0), size=min(2, M - b0), replace=False))
+                           for b0 in range(0, M, 32)])
+
+
+def write_outputs(directory, outputs):
+    """DIR/<workload>.npy, float32, for every workload the run timed (at most DUMP_LIMIT_BYTES in all)."""
+    import numpy as np
+    total = sum(a.nbytes for a in outputs.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(directory, exist_ok=True)
+    for name, arr in outputs.items():
+        np.save(os.path.join(directory, name + ".npy"), arr)
 
 
 def llama_weight_bytes():
@@ -380,6 +409,16 @@ class Bench:
         self.warm = max(args.warmup, 3)
         self.fused_note = None
         self._llama = None
+        self.last_out = None
+        self.outputs = {} if args.dump_outputs else None  # workload -> float32 array for --dump-outputs
+
+    def keep_output(self, name, y):
+        """--dump-outputs: a float32 host copy of the [M, N] result of workload `name`'s last timed step (the rows of
+        dump_rows(M)), taken right after its timed region."""
+        if self.outputs is None or self.rank != 0:
+            return
+        rows = torch.from_numpy(dump_rows(y.shape[0])).to(y.device)
+        self.outputs[name] = y.index_select(0, rows).float().cpu().numpy()
 
     # ---- timing -------------------------------------------------------------------------------------------------
     def barrier(self):
@@ -389,15 +428,16 @@ class Bench:
 
     def timed(self, step_fn, steps, warmup):
         """`steps` calls of step_fn(i) on the current stream between two CUDA events, bracketed by barrier +
-        synchronize; max over ranks.  Returns ms per step."""
+        synchronize; max over ranks.  Returns ms per step; what the last call returned is kept in `self.last_out`."""
         for i in range(warmup):
             step_fn(i)
         self.barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         self.sampler.active = True
         e0.record()
-        for i in range(steps):
+        for i in range(steps - 1):
             step_fn(warmup + i)
+        self.last_out = step_fn(warmup + steps - 1)
         e1.record()
         self.barrier()
         self.sampler.active = False
@@ -537,8 +577,9 @@ class Bench:
                 graphs.append(gr)
             rotation = torch.cuda.CUDAGraph()
             with torch.cuda.graph(rotation):
-                for c in range(n_copies):
+                for c in range(n_copies - 1):
                     gathered(x_dev, weights[c])
+                rotation_out = gathered(x_dev, weights[n_copies - 1])
 
         def step_device(i):
             if graphs is not None:
@@ -573,9 +614,12 @@ class Bench:
                     rotation.replay()
                 for c in range(rest):
                     graphs[c].replay()
+                return graph_outs[rest - 1] if rest else rotation_out
             ms_dev = self.timed(run_steps, 1, self.warm) / steps
         else:
             ms_dev = self.timed(step_device, steps, self.warm)
+        self.keep_output(name, self.last_out)
+        self.last_out = None  # not held through the next timed regions
         ms_e2e = self.timed(step_e2e, steps, self.warm)
         # roofline of the dominant kernel: the local shard's kernel alone (no gather), CUDA events on the launching stream
         if world == 1:
@@ -750,6 +794,7 @@ class Bench:
             y_host.copy_(out_g, non_blocking=True)
 
         ms_dev = self.timed(lambda i: graph.replay(), args.steps, self.warm)
+        self.keep_output(name, out_g)  # the graph's output buffer holds the last replay's result
         ms_e2e = self.timed(e2e_step, args.steps, self.warm)
         self.load_for_clocks(lambda i: graph.replay(), mark, max_seconds=1.0)
         clocks = self.sampler.snapshot(mark)
@@ -877,6 +922,8 @@ class Bench:
                 line["compare"] = self.compare_set()
             line["bench_seconds"] = round(time.time() - t_start, 1)
         self.sampler.stop()
+        if self.outputs is not None and self.rank == 0:
+            write_outputs(args.dump_outputs, self.outputs)
         if self.rank == 0:
             print(json.dumps(line))
         if self.world > 1:
@@ -893,7 +940,14 @@ def main():
     ap.add_argument("--gather", default="fused", choices=["fused", "nccl"],
                     help="multi-GPU int4: all-gather fused into the kernel (default) or kernel + NCCL all-gather")
     ap.add_argument("--no-extras", action="store_true", help="default workload only: skip the extra / compare sections")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the result of each timed workload's last step to "
+                         "DIR/<workload>.npy (float32; for M > 32 two seeded rows of every 32-row band)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of the GPU path (--impl ours)")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         if wl["kind"] == "llama":

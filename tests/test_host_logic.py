@@ -272,6 +272,25 @@ def test_bench_algorithmic_figures_match_the_scope_table():
     assert set(bench.WORKLOADS) >= {"qlinear_bf16_int4_m4096", "decode_m1", "int8_m4096", "llama3_8b_decode_b1"}
 
 
+def test_bench_dump_outputs_sample_and_files(tmp_path):
+    """bench.py --dump-outputs: small results are written whole, a large M as the same two rows of every 32-row band on
+    every run, as float32 .npy files, never more than 64 MB in all."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    assert np.array_equal(bench.dump_rows(32), np.arange(32))
+    rows = bench.dump_rows(4096)
+    assert len(rows) == 256 and np.all(np.diff(rows) > 0) and np.array_equal(np.bincount(rows // 32), np.full(128, 2))
+    assert np.array_equal(rows, bench.dump_rows(4096))
+    bench.write_outputs(str(tmp_path / "out"), {"decode_m1": np.ones((1, 8), np.float32)})
+    got = np.load(tmp_path / "out" / "decode_m1.npy")
+    assert got.dtype == np.float32 and got.shape == (1, 8)
+    with pytest.raises(SystemExit):
+        bench.write_outputs(str(tmp_path / "big"), {"x": np.zeros(bench.DUMP_LIMIT_BYTES // 4 + 1, np.float32)})
+    assert not (tmp_path / "big").exists()
+
+
 def test_qlinear_output_hook_passthrough_and_fused_forward_guards():
     """Host logic of the fused output quantisation (nn.py): the hook passes an already quantized output through, the
     fused forward declines CPU weights / unfrozen weights / a removed hook, and the hook bookkeeping follows removal."""
